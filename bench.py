@@ -49,6 +49,34 @@ CONFIGS = {   # BASELINE.json configs[1] and configs[2] (one GPU's share)
     "cfg3": dict(layers=24, embd=2048, batch=4, ctx=2048, name="RWKV-x070 1.5B (L24 C2048 H32 N64)"),
 }
 LORA_RANKS = {768: 64 + 64 + 32 + 128, 2048: 96 + 96 + 64 + 256}   # v7.00/src/model.py:118,127,133,140 (w, a, v, g)
+DUMP_SAMPLE = 16384   # elements written per tensor by --dump-outputs: ~24 MB for the 402 trainable tensors of cfg2
+
+
+def dump_outputs(out_dir, loss, named_params):
+    """What a caller of the timed step holds after its last step: the loss and, for every trainable parameter, its
+    gradient and its updated value, each as DIR/<kind>.<parameter name>.npy in float32.  A tensor of more than
+    DUMP_SAMPLE elements is reduced to a sample whose positions depend only on the parameter's name and size, so runs
+    with the same arguments (and therefore the same seeded inputs) can be compared file by file across builds.  Compare
+    with a tolerance: the bf16 gradients are not bitwise reproducible from run to run (at cfg2 on a B200 at 1000 W, two
+    runs of the same build differed by a median 0.7 % relative RMS over the gradient files, 1.7 % at most, with equal
+    losses)."""
+    import zlib
+
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    for name, p in named_params:
+        idx = None
+        if p.numel() > DUMP_SAMPLE:
+            g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+            idx = torch.randint(0, p.numel(), (DUMP_SAMPLE,), generator=g).to(p.device)
+        for kind, t in (("grad", p.grad), ("param", p)):
+            if t is None:
+                continue
+            flat = t.detach().reshape(-1)
+            if idx is not None:
+                flat = flat[idx]
+            np.save(os.path.join(out_dir, f"{kind}.{name}.npy"), flat.float().cpu().numpy())
 
 
 def load_peaks():
@@ -162,7 +190,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ref-kernel", action="store_true")
     ap.add_argument("--grad-cp", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss and a fixed sample of every trainable parameter's gradient and "
+                         "updated value from the last timed step to DIR/*.npy (float32)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[a.config]
     for k_ in ("batch", "ctx", "layers", "embd"):
         if getattr(a, k_) is None:
@@ -335,9 +368,16 @@ def main():
     if not graphed:
         wkv7.PROFILE = []
     lc0 = wkv7.launch_count()
+    last = {}
+
+    def timed_step():
+        last["loss"] = train_step(resident)
+
     with ClockSampler(local_rank) as cs:
-        ms = timed(lambda: train_step(resident), a.steps)
+        ms = timed(timed_step, a.steps)
     launches = wkv7.launch_count() - lc0
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, last["loss"], [(n, p) for n, p in model.named_parameters() if p.requires_grad])
     if graphed:
         # a replayed graph does not pass through the host-side launch counter, and CUDA events cannot time single kernels
         # inside it: count the launches of ONE eager replica of the step and time the WKV7 kernels there (same kernels,

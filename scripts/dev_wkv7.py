@@ -102,6 +102,9 @@ def timing(shape, fvs, bvs):
     return out
 
 
+REF_SLICE_SAMPLE = 8192
+
+
 def mint_golden(outdir):
     """Reference-kernel outputs for fixed seeds (the goldens tests/golden/ is built from)."""
     os.makedirs(outdir, exist_ok=True)
@@ -120,6 +123,39 @@ def mint_golden(outdir):
         np.savez_compressed(os.path.join(outdir, f"wkv7_ref_{name}.npz"), B=B, T=T, H=H, seed=seed,
                             kind=np.array(kind), **arrs)
         print("minted", name, {k2: v2.shape for k2, v2 in arrs.items()})
+
+    # the reference kernel's RMS error against the fp64 oracle, which our kernels must not exceed (full tensors)
+    B, T, H, seed = 2, 512, 4, 3
+    cpu = O.make_inputs(B, T, H, 64, seed=seed)
+    inp = [x.cuda() for x in cpu]
+    ry, rs, rsa = RK.forward(*inp[:6])
+    rg = RK.backward(*inp, rs, rsa)
+    torch.cuda.synchronize()
+    y64, s64, sa64 = O.forward(*cpu[:6])
+    g64 = O.backward(*cpu, s64, sa64)
+    errs = {"y": O.err_ratio(ry.float().cpu().numpy(), y64), "s": O.err_ratio(rs.cpu().numpy(), s64)}
+    for n, x, r in zip(["dw", "dq", "dk", "dv", "da", "db"], rg, g64):
+        errs[n] = O.err_ratio(x.float().cpu().numpy(), r)
+    np.savez(os.path.join(outdir, "wkv7_refkernel_errors_b2t512h4.npz"), B=B, T=T, H=H, seed=seed,
+             kind=np.array("realistic"), **errs)
+    print("minted reference errors", errs)
+
+    # the reference kernel on one (b, h) slice of the cfg2-size inputs, at a fixed sample of REF_SLICE_SAMPLE positions
+    # (every output of the slice has 2048 * 64 elements; the checkpoints kept are the chunk-end ones, rs[:, :, 3::4])
+    B, T, H, seed, bi, hi = 8, 2048, 12, 42, 3, 5
+    sub = [x[bi:bi + 1, :, hi:hi + 1].contiguous().cuda() for x in O.make_inputs(B, T, H, 64, seed=seed)]
+    ry, rs, rsa = RK.forward(*sub[:6])
+    rg = RK.backward(*sub, rs, rsa)
+    torch.cuda.synchronize()
+    idx = np.sort(np.random.default_rng(0).choice(T * 64, REF_SLICE_SAMPLE, replace=False)).astype(np.int32)
+    d = {"y": ry, "sa": rsa, "s": rs[:, :, 3::4].contiguous()}
+    for n, x in zip(["dw", "dq", "dk", "dv", "da", "db"], rg):
+        d[n] = x
+    arrs = {k2: (v2.view(torch.int16) if v2.dtype == torch.bfloat16 else v2).reshape(-1).cpu().numpy()[idx] for k2, v2 in d.items()}
+    rms = {"rms_" + n: float(torch.sqrt(torch.mean(x.double() ** 2))) for n, x in zip(["dw", "dq", "dk", "dv", "da", "db"], rg)}
+    np.savez_compressed(os.path.join(outdir, "wkv7_refkernel_slice_b8t2048h12.npz"), B=B, T=T, H=H, seed=seed, b=bi, h=hi,
+                        idx=idx, **arrs, **rms)
+    print("minted reference slice", {k2: v2.shape for k2, v2 in arrs.items()}, rms)
 
 
 if __name__ == "__main__":
