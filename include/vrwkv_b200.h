@@ -90,6 +90,21 @@ int vrwkv_wkv7_backward_ex(int B, int T, int H, const uint16_t* w, const uint16_
                            const uint16_t* b, const uint16_t* dy, const float* s, const float* sa,
                            uint16_t* dw, uint16_t* dq, uint16_t* dk, uint16_t* dv, uint16_t* da,
                            uint16_t* db, unsigned flags, void* stream);
+/* Chunk cache: with flags = BOUNDED_DECAY | CHUNK_CHECKPOINTS (T % 64 == 0, no carried state, s and sa required),
+ * forward_cache is forward_ex that also writes `cache`, and backward_cache is backward_ex that reads it back instead of
+ * recomputing what the forward already had: the masked 64x64 chunk matrices and the triangular inverse of each chunk.
+ * The cache holds vrwkv_wkv7_cache_bytes(B, T, H) bytes (64 KB per 64-step chunk of each (batch, head); 0 when
+ * T % 64 != 0), 128-byte aligned, and is only meaningful to backward_cache on the same inputs, s and sa. */
+size_t vrwkv_wkv7_cache_bytes(int B, int T, int H);
+int vrwkv_wkv7_forward_cache(int B, int T, int H, const uint16_t* w, const uint16_t* q,
+                             const uint16_t* k, const uint16_t* v, const uint16_t* a,
+                             const uint16_t* b, uint16_t* y, float* s, float* sa, void* cache,
+                             unsigned flags, void* stream);
+int vrwkv_wkv7_backward_cache(int B, int T, int H, const uint16_t* w, const uint16_t* q,
+                              const uint16_t* k, const uint16_t* v, const uint16_t* a,
+                              const uint16_t* b, const uint16_t* dy, const float* s, const float* sa,
+                              const void* cache, uint16_t* dw, uint16_t* dq, uint16_t* dk, uint16_t* dv,
+                              uint16_t* da, uint16_t* db, unsigned flags, void* stream);
 /* Synchronises the device and fails (VRWKV_EINVAL) if a chunked kernel saw decay outside the promised range since
  * the last check; the flag is cleared. */
 int vrwkv_wkv7_domain_check(void);

@@ -1,4 +1,5 @@
-"""Per-phase clock stamps of CTA 0's third work item in the x3 backward at cfg2 size."""
+"""Per-phase clock stamps of CTA 0's third work item in the x3 backward at cfg2 size (--cache: the variant that loads the
+forward's chunk cache; its stamps 1-3 coincide)."""
 import ctypes, os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -10,9 +11,13 @@ dbg = torch.zeros(4096, dtype=torch.float32, device="cuda")
 _lib.check(_lib.lib().vrwkv_wkv7_chunk_debug(ctypes.c_void_p(dbg.data_ptr())), "dbg")
 B, T, H = 8, 2048, 12
 w, q, k, v, a, b, dy = [x.cuda() for x in O.make_inputs(B, T, H, 64, seed=42)]
-y, s, sa = W.forward_raw(w, q, k, v, a, b, bounded_decay=True, chunk_checkpoints=True)
+cache = None
+if "--cache" in sys.argv:
+    y, s, sa, cache = W.forward_raw(w, q, k, v, a, b, bounded_decay=True, chunk_checkpoints=True, chunk_cache=True)
+else:
+    y, s, sa = W.forward_raw(w, q, k, v, a, b, bounded_decay=True, chunk_checkpoints=True)
 dbg.zero_()
-W.backward_raw(w, q, k, v, a, b, dy, s, sa, bounded_decay=True)
+W.backward_raw(w, q, k, v, a, b, dy, s, sa, bounded_decay=True, cache=cache)
 torch.cuda.synchronize()
 ts = [int(x) for x in dbg.cpu().numpy()[3072:3072 + 14]]
 d = [ts[i + 1] - ts[i] for i in range(13)]

@@ -10,13 +10,13 @@ dbg = torch.zeros(4096, dtype=torch.float32, device="cuda")
 _lib.check(_lib.lib().vrwkv_wkv7_chunk_debug(ctypes.c_void_p(dbg.data_ptr())), "dbg")
 B, T, H = 8, 2048, 12
 w, q, k, v, a, b, dy = [x.cuda() for x in O.make_inputs(B, T, H, 64, seed=42)]
-for ck in (True, False):
+for ck, cache in ((True, False), (False, False), (True, True)):
     W.set_variant(6, 0)
     dbg.zero_()
-    W.forward_raw(w, q, k, v, a, b, bounded_decay=True, chunk_checkpoints=ck)
+    W.forward_raw(w, q, k, v, a, b, bounded_decay=True, chunk_checkpoints=ck, chunk_cache=cache)
     torch.cuda.synchronize()
     ts = [int(x) for x in dbg.cpu().numpy()[2048:2048 + 17]]
     d = [ts[i + 1] - ts[i] for i in range(16)]
-    print("ck64" if ck else "ck16", "total", ts[16], " ".join(f"{n}={x}" for n, x in zip(names, d)))
+    print("ck64+cache" if cache else "ck64" if ck else "ck16", "total", ts[16], " ".join(f"{n}={x}" for n, x in zip(names, d)))
 W.set_variant(0, 0)
 _lib.check(_lib.lib().vrwkv_wkv7_chunk_debug(ctypes.c_void_p(0)), "dbg")

@@ -90,6 +90,12 @@ __device__ __forceinline__ void bulk_load_1d(void* dst, const void* src, uint32_
         "l"(reinterpret_cast<uint64_t>(src)), "r"(bytes), "r"(smem_u32(bar))
         : "memory");
 }
+// 1-D bulk copy shared -> global (bulk group completion: tma_store_commit / tma_store_wait*).
+__device__ __forceinline__ void bulk_store_1d(void* dst, const void* src, uint32_t bytes) {
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(reinterpret_cast<uint64_t>(dst)),
+                 "r"(smem_u32(src)), "r"(bytes)
+                 : "memory");
+}
 
 // ---------------------------------------------------------------------------------------------
 // packed fp32x2 arithmetic (Blackwell FFMA2 / FMUL2 / FADD2)

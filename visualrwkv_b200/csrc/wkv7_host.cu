@@ -166,8 +166,9 @@ static int make_tile_map(CUtensorMap* m, const void* base, int B, int T, int H) 
                            (uint64_t)H * WKV_N * 2, WKV_N, X6_L, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
-// round-2 forward: chunk-parallel persistent kernel, x6 products (wkv7_x6_fwd.cuh)
-static int launch_x6_fwd(const void* const* in, const Wkv7FwdArgs& a, bool chunk_ck, cudaStream_t st) {
+// round-2 forward: chunk-parallel persistent kernel, x6 products (wkv7_x6_fwd.cuh); `cache` (chunk checkpoints only):
+// also write the chunk cache
+static int launch_x6_fwd(const void* const* in, const Wkv7FwdArgs& a, bool chunk_ck, cudaStream_t st, void* cache = nullptr) {
     int rc = ensure_pool_keeps_memory();
     if (rc) return rc;
     CUtensorMap tm[6];
@@ -179,10 +180,11 @@ static int launch_x6_fwd(const void* const* in, const Wkv7FwdArgs& a, bool chunk
     uint8_t* ws = nullptr;
     VRWKV_CUDA(cudaMallocAsync((void**)&ws, sync_bytes + chain_bytes, st));
     VRWKV_CUDA(cudaMemsetAsync(ws, 0, sync_bytes, st));
-    X6FwdArgs xa{a.B, a.T, a.H, a.y, a.s, a.sa, a.state_in, a.state_out, chain_bytes ? (float*)(ws + sync_bytes) : nullptr, (int*)ws};
+    X6FwdArgs xa{a.B, a.T, a.H, a.y, a.s, a.sa, a.state_in, a.state_out, chain_bytes ? (float*)(ws + sync_bytes) : nullptr, (int*)ws,
+                 (uint8_t*)cache};
     const size_t smem = sizeof(X6FwdSmem) + 1024;
     // 16-step checkpoints only when a checkpoint tensor in the reference's layout was asked for
-    auto kern = (chunk_ck || !a.s) ? wkv7_x6_fwd_kernel<false> : wkv7_x6_fwd_kernel<true>;
+    auto kern = cache ? wkv7_x6_fwd_kernel<false, true> : (chunk_ck || !a.s) ? wkv7_x6_fwd_kernel<false> : wkv7_x6_fwd_kernel<true>;
     VRWKV_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int grid = nitems < sm_count() ? nitems : sm_count();
     kern<<<grid, X6_THREADS, smem, st>>>(tm[0], tm[1], tm[2], tm[3], tm[4], tm[5], xa);
@@ -192,10 +194,10 @@ static int launch_x6_fwd(const void* const* in, const Wkv7FwdArgs& a, bool chunk
     return VRWKV_OK;
 }
 
-// round-2 backward: one chunk-parallel persistent kernel, x3 products (wkv7_x6_bwd.cuh)
+// round-2 backward: one chunk-parallel persistent kernel, x3 products (wkv7_x6_bwd.cuh); `cache`: the forward's chunk cache
 static int launch_x3_bwd(const uint16_t* w, const uint16_t* q, const uint16_t* k, const uint16_t* v, const uint16_t* a,
                          const uint16_t* b, const uint16_t* dy, const float* sa, const Wkv7BwdArgs& args, int ck_per_chunk,
-                         cudaStream_t st) {
+                         cudaStream_t st, const void* cache = nullptr) {
     int rc = ensure_pool_keeps_memory();
     if (rc) return rc;
     const int B = args.B, T = args.T, H = args.H;
@@ -210,11 +212,12 @@ static int launch_x3_bwd(const uint16_t* w, const uint16_t* q, const uint16_t* k
     VRWKV_CUDA(cudaMallocAsync((void**)&ws, sync_bytes + ring_bytes, st));
     VRWKV_CUDA(cudaMemsetAsync(ws, 0, sync_bytes, st));
     X3BwdArgs xa{B, T, H, w, q, k, a, b, sa, args.s, ck_per_chunk, (float*)(ws + sync_bytes), (int*)ws,
-                 args.dw, args.dq, args.dk, args.dv, args.da, args.db};
+                 args.dw, args.dq, args.dk, args.dv, args.da, args.db, (const uint8_t*)cache};
     const size_t smem = sizeof(X3BwdSmem) + 1024;
-    VRWKV_CUDA(cudaFuncSetAttribute(wkv7_x3_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    auto kern = cache ? wkv7_x3_bwd_kernel<true> : wkv7_x3_bwd_kernel<false>;
+    VRWKV_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int grid = nitems < sm_count() ? nitems : sm_count();
-    wkv7_x3_bwd_kernel<<<grid, X6_THREADS, smem, st>>>(tm[0], tm[1], tm[2], tm[3], tm[4], tm[5], tm[6], xa);
+    kern<<<grid, X6_THREADS, smem, st>>>(tm[0], tm[1], tm[2], tm[3], tm[4], tm[5], tm[6], xa);
     VRWKV_CUDA(cudaGetLastError());
     vrwkv_count_launch(1);
     VRWKV_CUDA(cudaFreeAsync(ws, st));
@@ -370,4 +373,44 @@ extern "C" int vrwkv_wkv7_backward(int B, int T, int H, const uint16_t* w, const
                                    const float* s, const float* sa, uint16_t* dw, uint16_t* dq, uint16_t* dk,
                                    uint16_t* dv, uint16_t* da, uint16_t* db, void* stream) {
     return vrwkv_wkv7_backward_ex(B, T, H, w, q, k, v, a, b, dy, s, sa, dw, dq, dk, dv, da, db, 0u, stream);
+}
+
+// ---- chunk cache (model path) ----
+static const unsigned kCacheFlags = VRWKV_WKV7_BOUNDED_DECAY | VRWKV_WKV7_CHUNK_CHECKPOINTS;
+
+extern "C" size_t vrwkv_wkv7_cache_bytes(int B, int T, int H) {
+    if (B <= 0 || T <= 0 || H <= 0 || T % X6_L) return 0;
+    return (size_t)B * H * (T / X6_L) * XC_ITEM_BYTES;
+}
+
+static int check_cache_call(const char* what, int T, const void* s, const void* sa, const void* cache, unsigned flags) {
+    if ((flags & (kCacheFlags | VRWKV_WKV7_TF32)) != kCacheFlags)
+        return vrwkv_fail(VRWKV_EINVAL, "%s: needs flags BOUNDED_DECAY | CHUNK_CHECKPOINTS (and not TF32), got 0x%x", what, flags);
+    if (T % X6_L) return vrwkv_fail(VRWKV_EINVAL, "%s: T=%d must be a multiple of %d", what, T, X6_L);
+    if (!s || !sa || !cache) return vrwkv_fail(VRWKV_EINVAL, "%s: s, sa and cache are required", what);
+    if (((uintptr_t)s | (uintptr_t)sa) & 15) return vrwkv_fail(VRWKV_EINVAL, "%s: s and sa must be 16-byte aligned", what);
+    if ((uintptr_t)cache & 127) return vrwkv_fail(VRWKV_EINVAL, "%s: cache must be 128-byte aligned", what);
+    return VRWKV_OK;
+}
+
+extern "C" int vrwkv_wkv7_forward_cache(int B, int T, int H, const uint16_t* w, const uint16_t* q, const uint16_t* k,
+                                        const uint16_t* v, const uint16_t* a, const uint16_t* b, uint16_t* y, float* s,
+                                        float* sa, void* cache, unsigned flags, void* stream) {
+    const void* ptrs[] = {w, q, k, v, a, b, y};
+    int rc = check_common(B, T, H, ptrs, 7);
+    if (rc || (rc = check_cache_call("wkv7 forward_cache", T, s, sa, cache, flags))) return rc;
+    const void* in[6] = {w, q, k, v, a, b};
+    Wkv7FwdArgs args{B, T, H, y, s, sa, nullptr, nullptr};
+    return launch_x6_fwd(in, args, true, (cudaStream_t)stream, cache);
+}
+
+extern "C" int vrwkv_wkv7_backward_cache(int B, int T, int H, const uint16_t* w, const uint16_t* q, const uint16_t* k,
+                                         const uint16_t* v, const uint16_t* a, const uint16_t* b, const uint16_t* dy,
+                                         const float* s, const float* sa, const void* cache, uint16_t* dw, uint16_t* dq,
+                                         uint16_t* dk, uint16_t* dv, uint16_t* da, uint16_t* db, unsigned flags, void* stream) {
+    const void* ptrs[] = {w, q, k, v, a, b, dy, s, sa, dw, dq, dk, dv, da, db};
+    int rc = check_common(B, T, H, ptrs, 15);
+    if (rc || (rc = check_cache_call("wkv7 backward_cache", T, s, sa, cache, flags))) return rc;
+    Wkv7BwdArgs args{B, T, H, s, dw, dq, dk, dv, da, db};
+    return launch_x3_bwd(w, q, k, v, a, b, dy, sa, args, 1, (cudaStream_t)stream, cache);
 }

@@ -30,6 +30,7 @@ struct X3BwdArgs {
     float* ds;                           // [B*H][2][64*64] ring of dL/dS (row-major [i][j])
     int* sync;                           // [0] item counter, [1 + bh] chunks finished (from the end); zeroed before launch
     uint16_t *dw, *dq, *dk, *dv, *da, *db;
+    const uint8_t* cache;                // CACHE: the forward's chunk cache, [B*H*T/64][8 tiles][8 KB] (wkv7_x6_common.cuh)
 };
 
 struct alignas(1024) X3BwdSmem {
@@ -47,8 +48,13 @@ struct alignas(1024) X3BwdSmem {
     uint64_t bar_in, bar_dy, bar_v, bar_mma, bar_c3;
     uint32_t tmem_base;
     int next_item;
+    uint64_t bar_ca;              // CACHE: the item's chunk-cache tiles
 };
 
+// CACHE: [A_qb|A_qk], A_ak and Tinv come from the forward's chunk cache instead of the scores batch, P2 and the inverse.
+// They land in r2, sak and the dR slots of drdy (Tinv part p at p*16384), all dead once the item's dA batch has finished,
+// so the next item's cache loads are issued there, together with its raw-input loads.
+template <bool CACHE = false>
 __global__ void __launch_bounds__(X6_THREADS, 1)
 wkv7_x3_bwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_q,
                    const __grid_constant__ CUtensorMap tm_k, const __grid_constant__ CUtensorMap tm_v,
@@ -76,6 +82,7 @@ wkv7_x3_bwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_consta
         mbar_init(&sm.bar_v, 1);
         mbar_init(&sm.bar_mma, 1);
         mbar_init(&sm.bar_c3, 1);
+        if constexpr (CACHE) mbar_init(&sm.bar_ca, 1);
         fence_mbar_init();
         tma_prefetch_desc(&tm_w); tma_prefetch_desc(&tm_q); tma_prefetch_desc(&tm_k); tma_prefetch_desc(&tm_v);
         tma_prefetch_desc(&tm_a); tma_prefetch_desc(&tm_b); tma_prefetch_desc(&tm_dy);
@@ -129,11 +136,25 @@ wkv7_x3_bwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_consta
         mbar_arrive_expect_tx(&sm.bar_v, BT_BYTES);
         tma_load_2d(sm.r2 + BT_BYTES, &tm_v, hh * N, bb * T + c * L, &sm.bar_v);
     };
+    auto load_cache = [&](int item) {
+        int c, bh, bb, hh;
+        item_coords(item, c, bh, bb, hh);
+        const uint8_t* src = p.cache + (size_t)(c * BH + bh) * XC_ITEM_BYTES;
+        mbar_arrive_expect_tx(&sm.bar_ca, XC_ITEM_BYTES);
+        bulk_load_1d(sm.r2, src + XC_QB0 * BT_BYTES, 4 * BT_BYTES, &sm.bar_ca);   // [A_qb|A_qk] pairs, part p at p*16384
+        bulk_load_1d(sm.sak, src + XC_AK0 * BT_BYTES, 2 * BT_BYTES, &sm.bar_ca);
+        bulk_load_1d(sm.drdy, src + XC_TI0 * BT_BYTES, BT_BYTES, &sm.bar_ca);
+        bulk_load_1d(sm.drdy + 16384, src + XC_TI1 * BT_BYTES, BT_BYTES, &sm.bar_ca);
+    };
     int item = sm.next_item;
-    if (tid == 0 && item < nitems) { load_in5(item); load_dy(item); }
+    if (tid == 0 && item < nitems) {
+        load_in5(item);
+        load_dy(item);
+        if constexpr (CACHE) load_cache(item);
+    }
     __syncwarp();
 
-    uint32_t ph_in = 0, ph_dy = 0, ph_v = 0, ph_mma = 0, ph_c3 = 0;
+    uint32_t ph_in = 0, ph_dy = 0, ph_v = 0, ph_mma = 0, ph_c3 = 0, ph_ca = 0;
 #ifdef VRWKV_PHASE_STAMPS   // development aid (scripts/dbg_x6_stamps.py, dbg_x3_stamps.py): build with VRWKV_PHASE_STAMPS=1
     float* const dbg = (blockIdx.x == 0 && tid == 0) ? g_chunk_dbg : nullptr;
     int lt = 0, tsi = 0;
@@ -238,69 +259,88 @@ wkv7_x3_bwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_consta
         }
         operands_ready();
         stamp();  // 1
-        // ================= scores = [At;Qt] [Bt;Kt]^T =================
-        if (warp == 0) {
-            if (elect_one()) {
-                tc_fence_after();
-                mma_x3<128, 0, 0>(tmem + C_SC, b4, O_AQ, 16384, O_BK, 16384, false);
-                umma_commit(&sm.bar_mma);
-            }
-            __syncwarp();
-        }
-        mma_wait();
-        stamp();  // 2
-        // ================= P2: masked scores: A_ab fp32 (inverse), [A_qb|A_qk] and A_ak operands =================
-        {
-            uint32_t v[32];
-            tmem_ld32(tm_row + C_SC + 32 * cs, v);
-            const int tq = r & 63;
-            const bool incl = r >= 64;
-            float o[32];
-#pragma unroll
-            for (int e = 0; e < 32; e++) {
-                const int s = 32 * (cs & 1) + e;
-                const bool keep = incl ? (s <= tq) : (s < tq);
-                o[e] = keep ? __uint_as_float(v[e]) : 0.f;
-            }
-            if (incl) {   // q rows: A_qb (cs 0,1) -> r2 tile 0, A_qk (cs 2,3) -> r2 tile 1
-                uint8_t* dst = sm.r2 + (cs >> 1) * BT_BYTES;
-#pragma unroll
-                for (int cc = 0; cc < 4; cc++) {
-                    const float x8[8] = {o[8 * cc], o[8 * cc + 1], o[8 * cc + 2], o[8 * cc + 3], o[8 * cc + 4], o[8 * cc + 5], o[8 * cc + 6], o[8 * cc + 7]};
-                    store_pair8(dst + bt_chunk(tq, 4 * (cs & 1) + cc), 16384, x8);
+        if constexpr (CACHE) {
+            stamp();  // 2
+            stamp();  // 3
+            // ================= [dU;dV] = [A_qb|A_qk]^T dY with the forward's tiles =================
+            if (warp == 0) {
+                mbar_wait(&sm.bar_ca, ph_ca & 1);
+                mbar_wait(&sm.bar_dy, ph_dy & 1);
+                if (elect_one()) {
+                    tc_fence_after();
+                    mma_x2b<64, 1, 1>(tmem + C_UV, b4, O_R2, 16384, O_DRDY + BT_BYTES, false);
+                    umma_commit(&sm.bar_mma);
                 }
-            } else if (cs < 2) {   // A_ab
+                __syncwarp();
+            }
+            ph_ca++;
+            ph_dy++;
+            mma_wait();
+        } else {
+            // ================= scores = [At;Qt] [Bt;Kt]^T =================
+            if (warp == 0) {
+                if (elect_one()) {
+                    tc_fence_after();
+                    mma_x3<128, 0, 0>(tmem + C_SC, b4, O_AQ, 16384, O_BK, 16384, false);
+                    umma_commit(&sm.bar_mma);
+                }
+                __syncwarp();
+            }
+            mma_wait();
+            stamp();  // 2
+            // ================= P2: masked scores: A_ab fp32 (inverse), [A_qb|A_qk] and A_ak operands =================
+            {
+                uint32_t v[32];
+                tmem_ld32(tm_row + C_SC + 32 * cs, v);
+                const int tq = r & 63;
+                const bool incl = r >= 64;
+                float o[32];
 #pragma unroll
-                for (int cc = 0; cc < 8; cc++) *m64_chunk(mab, r, 8 * cs + cc) = make_float4(o[4 * cc], o[4 * cc + 1], o[4 * cc + 2], o[4 * cc + 3]);
-            } else {               // A_ak
+                for (int e = 0; e < 32; e++) {
+                    const int s = 32 * (cs & 1) + e;
+                    const bool keep = incl ? (s <= tq) : (s < tq);
+                    o[e] = keep ? __uint_as_float(v[e]) : 0.f;
+                }
+                if (incl) {   // q rows: A_qb (cs 0,1) -> r2 tile 0, A_qk (cs 2,3) -> r2 tile 1
+                    uint8_t* dst = sm.r2 + (cs >> 1) * BT_BYTES;
 #pragma unroll
-                for (int cc = 0; cc < 4; cc++) {
-                    const float x8[8] = {o[8 * cc], o[8 * cc + 1], o[8 * cc + 2], o[8 * cc + 3], o[8 * cc + 4], o[8 * cc + 5], o[8 * cc + 6], o[8 * cc + 7]};
-                    store_pair8(sm.sak + bt_chunk(r, 4 * (cs & 1) + cc), BT_BYTES, x8);
+                    for (int cc = 0; cc < 4; cc++) {
+                        const float x8[8] = {o[8 * cc], o[8 * cc + 1], o[8 * cc + 2], o[8 * cc + 3], o[8 * cc + 4], o[8 * cc + 5], o[8 * cc + 6], o[8 * cc + 7]};
+                        store_pair8(dst + bt_chunk(tq, 4 * (cs & 1) + cc), 16384, x8);
+                    }
+                } else if (cs < 2) {   // A_ab
+#pragma unroll
+                    for (int cc = 0; cc < 8; cc++) *m64_chunk(mab, r, 8 * cs + cc) = make_float4(o[4 * cc], o[4 * cc + 1], o[4 * cc + 2], o[4 * cc + 3]);
+                } else {               // A_ak
+#pragma unroll
+                    for (int cc = 0; cc < 4; cc++) {
+                        const float x8[8] = {o[8 * cc], o[8 * cc + 1], o[8 * cc + 2], o[8 * cc + 3], o[8 * cc + 4], o[8 * cc + 5], o[8 * cc + 6], o[8 * cc + 7]};
+                        store_pair8(sm.sak + bt_chunk(r, 4 * (cs & 1) + cc), BT_BYTES, x8);
+                    }
                 }
             }
-        }
-        mbar_wait(&sm.bar_dy, ph_dy & 1);
-        ph_dy++;
-        operands_ready();
-        stamp();  // 3
-        // ================= [dU;dV] = [A_qb|A_qk]^T dY   (inverse meanwhile) =================
-        if (warp == 0) {
-            if (elect_one()) {
-                tc_fence_after();
-                mma_x2b<64, 1, 1>(tmem + C_UV, b4, O_R2, 16384, O_DRDY + BT_BYTES, false);
-                umma_commit(&sm.bar_mma);
+            mbar_wait(&sm.bar_dy, ph_dy & 1);
+            ph_dy++;
+            operands_ready();
+            stamp();  // 3
+            // ================= [dU;dV] = [A_qb|A_qk]^T dY   (inverse meanwhile) =================
+            if (warp == 0) {
+                if (elect_one()) {
+                    tc_fence_after();
+                    mma_x2b<64, 1, 1>(tmem + C_UV, b4, O_R2, 16384, O_DRDY + BT_BYTES, false);
+                    umma_commit(&sm.bar_mma);
+                }
+                __syncwarp();
             }
-            __syncwarp();
+            tri_inverse_inplace(mab, sm.esc, reinterpret_cast<float*>(tinv), tid);
+            {   // Tinv pair [t][s]
+                const int t = tid >> 3, ch = tid & 7;
+                const float4 lo = *m64_chunk(mab, t, 2 * ch), hi = *m64_chunk(mab, t, 2 * ch + 1);
+                const float x8[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
+                store_pair8(tinv + bt_chunk(t, ch), BT_BYTES, x8);
+            }
+            mma_wait();
         }
-        tri_inverse_inplace(mab, sm.esc, reinterpret_cast<float*>(tinv), tid);
-        {   // Tinv pair [t][s]
-            const int t = tid >> 3, ch = tid & 7;
-            const float4 lo = *m64_chunk(mab, t, 2 * ch), hi = *m64_chunk(mab, t, 2 * ch + 1);
-            const float x8[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
-            store_pair8(tinv + bt_chunk(t, ch), BT_BYTES, x8);
-        }
-        mma_wait();
         stamp();  // 4
         // r2 is free: v tile, zero tile, next item's raw tiles cannot start yet (r1 holds Tinv)
         if (tid == 0) load_v(item);
@@ -377,7 +417,8 @@ wkv7_x3_bwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_consta
         if (warp == 0) {
             if (elect_one()) {
                 tc_fence_after();
-                mma_x3<64, 1, 1>(tmem + C_R, b4, O_TINV, BT_BYTES, O_DU, BT_BYTES, false);
+                if constexpr (CACHE) mma_x3<64, 1, 1>(tmem + C_R, b4, O_DRDY, 16384, O_DU, BT_BYTES, false);
+                else mma_x3<64, 1, 1>(tmem + C_R, b4, O_TINV, BT_BYTES, O_DU, BT_BYTES, false);
                 umma_commit(&sm.bar_mma);
             }
             __syncwarp();
@@ -476,7 +517,10 @@ wkv7_x3_bwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_consta
         if (tid == 0) {
             const int nxt = atomicAdd(&p.sync[0], 1);
             sm.next_item = nxt;
-            if (nxt < nitems) load_in5(nxt);
+            if (nxt < nitems) {
+                load_in5(nxt);
+                if constexpr (CACHE) load_cache(nxt);
+            }
         }
         // ================= P6: dA and dA^T masked, packed to bf16 pairs in place in TMEM (A operands) =================
         {

@@ -23,6 +23,13 @@ constexpr int X6_THREADS = 512;   // 16 warps: TMEM lane quadrant = warp & 3, co
 constexpr uint32_t X6_TRIPLE64 = 3 * BT_BYTES;       // 3 parts of one 64-row tile
 constexpr uint32_t X6_TRIPLE128 = 3 * 2 * BT_BYTES;  // 3 parts of a 128-row operand (two tiles per part)
 
+// Chunk cache (model path): tiles the forward holds anyway and the backward would otherwise rebuild — the masked chunk
+// matrices A_qb, A_qk, A_ak and Tinv = (I - A_ab)^-1 — as byte images of the shared-memory tiles ([t][s], SWIZZLE_128B).
+// Parts 0 and 1 of the forward's three-way split are exactly the backward's two-way split (split3x2 begins with the
+// two cvt.rn steps of split2x2).  Per item (chunk c of (b,h), stored at item c * B*H + b*H + h) 8 tiles of 8 KB:
+constexpr uint32_t XC_QB0 = 0, XC_QK0 = 1, XC_QB1 = 2, XC_QK1 = 3, XC_AK0 = 4, XC_AK1 = 5, XC_TI0 = 6, XC_TI1 = 7;
+constexpr uint32_t XC_ITEM_BYTES = 8 * BT_BYTES;
+
 __device__ __forceinline__ bool elect_one() {
     uint32_t pred;
     asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));

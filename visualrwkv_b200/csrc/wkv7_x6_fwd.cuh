@@ -54,9 +54,11 @@ struct X6FwdArgs {
     float* state_out;         // may be null
     float* chain;             // used when s == null: [B*H][2][64*64] hand-off buffer (transposed states)
     int* sync;                // [0] item counter, [1 + b*H + h] number of finished chunks of (b,h); zeroed before launch
+    uint8_t* cache;           // CACHE: the chunk cache, [B*H*T/64][8 tiles][8 KB] (wkv7_x6_common.cuh)
 };
 
-template <bool CK16>
+// CACHE: also write every item's chunk-cache tiles with 1-D bulk copies, each as soon as its tile exists (model path only).
+template <bool CK16, bool CACHE = false>
 __global__ void __launch_bounds__(X6_THREADS, 1)
 wkv7_x6_fwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_q,
                    const __grid_constant__ CUtensorMap tm_k, const __grid_constant__ CUtensorMap tm_v,
@@ -98,6 +100,8 @@ wkv7_x6_fwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_consta
                    O_BK = (uint32_t)(sm.bk - (uint8_t*)&sm), O_SCA = (uint32_t)(sm.sca - (uint8_t*)&sm), O_AVU = (uint32_t)(sm.avu - (uint8_t*)&sm);
     const uint32_t O_TINV = O_IN + 16384;
 
+    // the cache stores are issued and drained by one thread of warp 2, which idles in the inverse's diagonal blocks
+    constexpr int XC_TID = 64;
     auto load_in5 = [&](int item) {   // w,q,k,a,b tiles of an item (one thread)
         const int c = item / BH, bh = item - c * BH, bb = bh / H, hh = bh - bb * H;
         const int x0 = hh * N, y0 = bb * T + c * L;
@@ -258,6 +262,17 @@ wkv7_x6_fwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_consta
         ph_v++;
         operands_ready();
         stamp();  // 4: P2 done
+        if constexpr (CACHE) {
+            if (tid == XC_TID) {   // [A_ak;A_qk] parts 0 and 1: drained before the inverse's first barrier, so before P3 reuses sca
+                uint8_t* dst = p.cache + (size_t)item * XC_ITEM_BYTES;
+                bulk_store_1d(dst + XC_AK0 * BT_BYTES, sm.sca, BT_BYTES);
+                bulk_store_1d(dst + XC_QK0 * BT_BYTES, sm.sca + BT_BYTES, BT_BYTES);
+                bulk_store_1d(dst + XC_AK1 * BT_BYTES, sm.sca + 16384, BT_BYTES);
+                bulk_store_1d(dst + XC_QK1 * BT_BYTES, sm.sca + 16384 + BT_BYTES, BT_BYTES);
+                tma_store_commit();
+                tma_store_wait_read<0>();
+            }
+        }
         // ================= ACC = [A_ak;A_qk] V (runs while the inverse is being computed) =================
         if (warp == 0) {
             if (elect_one()) {
@@ -298,6 +313,15 @@ wkv7_x6_fwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_consta
         }
         operands_ready();
         stamp();  // 6: P3 done
+        if constexpr (CACHE) {
+            if (tid == XC_TID) {   // A_qb parts 0 and 1, Tinv parts 0 and 1: read while the W batch runs
+                uint8_t* dst = p.cache + (size_t)item * XC_ITEM_BYTES;
+                bulk_store_1d(dst + XC_QB0 * BT_BYTES, sm.sca + BT_BYTES, BT_BYTES);
+                bulk_store_1d(dst + XC_QB1 * BT_BYTES, sm.sca + 16384 + BT_BYTES, BT_BYTES);
+                bulk_store_1d(dst + XC_TI0 * BT_BYTES, tinv, 2 * BT_BYTES);
+                tma_store_commit();
+            }
+        }
         // ================= W = [A_ab;A_qb] Tinv =================
         if (warp == 0) {
             if (elect_one()) {
@@ -309,6 +333,10 @@ wkv7_x6_fwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_consta
         }
         mma_wait();
         stamp();  // 7: W done
+        if constexpr (CACHE) {   // P4 overwrites sca and the next item's loads overwrite Tinv
+            if (tid == XC_TID) tma_store_wait_read<0>();
+            __syncthreads();
+        }
         // the raw-input buffer (M / Tinv) is dead: fetch the next item and start its loads
         if (tid == 0) {
             const int nxt = atomicAdd(&p.sync[0], 1);
@@ -519,6 +547,9 @@ wkv7_x6_fwd_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_consta
         if (tid == 0) st_release(p.sync + 1 + bh, c + 1);
         stamp();  // 16: item done
         lt++;
+    }
+    if constexpr (CACHE) {
+        if (tid == XC_TID) tma_store_wait<0>();
     }
     tc_fence_before();
     __syncthreads();

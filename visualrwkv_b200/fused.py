@@ -179,16 +179,21 @@ def set_wkv_path(path: str) -> None:
 
 
 def wkv7_fwd_raw(w, q, k, v, a, b):
-    """[B,T,H,64] bf16 x6 -> y, s, sa."""
+    """[B,T,H,64] bf16 x6 -> y, s, sa, cache (the x6 path's chunk cache for wkv7_bwd_raw; None on the other paths)."""
     if WKV_PATH == "tf32":
-        return _wkv7.forward_raw(w, q, k, v, a, b, bounded_decay=True, chunk_checkpoints=True, tf32=True)
+        return (*_wkv7.forward_raw(w, q, k, v, a, b, bounded_decay=True, chunk_checkpoints=True, tf32=True), None)
     if WKV_PATH == "x6":
-        return _wkv7.forward_raw(w, q, k, v, a, b, bounded_decay=True, chunk_checkpoints=X3_BACKWARD)
-    return _wkv7.forward_raw(w, q, k, v, a, b)
+        if X3_BACKWARD and w.shape[1] % _wkv7.CHUNK == 0:
+            # the backward then loads each chunk's masked matrices and inverse instead of recomputing them (other T take
+            # the step-by-step kernels, which have no cache)
+            return _wkv7.forward_raw(w, q, k, v, a, b, bounded_decay=True, chunk_checkpoints=True, chunk_cache=True)
+        return (*_wkv7.forward_raw(w, q, k, v, a, b, bounded_decay=True), None)
+    return (*_wkv7.forward_raw(w, q, k, v, a, b), None)
 
 
-def wkv7_bwd_raw(w, q, k, v, a, b, dy, s, sa):
-    return _wkv7.backward_raw(w, q, k, v, a, b, dy, s, sa, bounded_decay=(WKV_PATH != "step"), tf32=(WKV_PATH == "tf32"))
+def wkv7_bwd_raw(w, q, k, v, a, b, dy, s, sa, cache=None):
+    return _wkv7.backward_raw(w, q, k, v, a, b, dy, s, sa, bounded_decay=(WKV_PATH != "step"), tf32=(WKV_PATH == "tf32"),
+                              cache=cache)
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -266,14 +271,14 @@ class TmixBlockFn(torch.autograd.Function):
                                                 v0.reshape(C) if has_vres else None, k_k.reshape(C), k_a.reshape(C))
         H = n_head
         v4 = lambda t: t.view(B, T, H, 64)
-        y, s, sa = wkv7_fwd_raw(v4(w), v4(r), v4(k2), v4(v2_), v4(nkk), v4(kka))
+        y, s, sa, wcache = wkv7_fwd_raw(v4(w), v4(r), v4(k2), v4(v2_), v4(nkk), v4(kka))
         z = tmix_post_forward(y.view(rows, C), r, k2, v2_, g, lnx_w, lnx_b, r_k.reshape(C), gn_eps)
         if own:
             out = gemm2(z, Wo, G2_TN, EPI_ADD, x2) if with_ln else gemm2(z, Wo)
         else:
             out = torch.addmm(x2, z, Wo.t()) if with_ln else z @ Wo.t()
         ctx.save_for_backward(x2, stats, ln_w, ln_b, *coefs, xr, xw, xk, xv, xa, xg, r, k, v, hw, ww, ha, aa, hg, g, hv, vv, vf2,
-                              w, k2, v2_, nkk, kka, y, s, sa, z, w0, w1, w2, a0, a1, a2, v0, v1, v2, g1, g2, k_k, k_a, r_k,
+                              w, k2, v2_, nkk, kka, y, s, sa, wcache, z, w0, w1, w2, a0, a1, a2, v0, v1, v2, g1, g2, k_k, k_a, r_k,
                               Wr, Wk, Wv, Wo, lnx_w, lnx_b)
         ctx.meta = (B, T, C, H, layer_id, ln_eps, gn_eps, with_ln)
         ctx.lora_own = lora_own
@@ -285,8 +290,8 @@ class TmixBlockFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dout, dvfirst_out):
         (x2, stats, ln_w, ln_b, c_r, c_w, c_k, c_v, c_a, c_g, xr, xw, xk, xv, xa, xg, r, k, v, hw, ww, ha, aa, hg, g, hv, vv, vf2,
-         w, k2, v2_, nkk, kka, y, s, sa, z, w0, w1, w2, a0, a1, a2, v0, v1, v2, g1, g2, k_k, k_a, r_k, Wr, Wk, Wv, Wo, lnx_w,
-         lnx_b) = ctx.saved_tensors
+         w, k2, v2_, nkk, kka, y, s, sa, wcache, z, w0, w1, w2, a0, a1, a2, v0, v1, v2, g1, g2, k_k, k_a, r_k, Wr, Wk, Wv, Wo,
+         lnx_w, lnx_b) = ctx.saved_tensors
         B, T, C, H, layer_id, ln_eps, gn_eps, with_ln = ctx.meta
         rows = B * T
         has_vres = layer_id != 0
@@ -295,7 +300,7 @@ class TmixBlockFn(torch.autograd.Function):
         dz = gemm2(do, Wo, G2_NN) if own else do @ Wo
         dy, dr, dk2a, dv2a, dg, red3 = tmix_post_backward(y.view(rows, C), r, k2, v2_, g, lnx_w, lnx_b, r_k.reshape(C), gn_eps, dz)
         v4 = lambda t: t.view(B, T, H, 64)
-        dw, dq, dk2b, dv2b, dnkk, dkka = wkv7_bwd_raw(v4(w), v4(r), v4(k2), v4(v2_), v4(nkk), v4(kka), v4(dy), s, sa)
+        dw, dq, dk2b, dv2b, dnkk, dkka = wkv7_bwd_raw(v4(w), v4(r), v4(k2), v4(v2_), v4(nkk), v4(kka), v4(dy), s, sa, wcache)
         dr.add_(dq.view(rows, C))
         dk, dv, dvf, dww, daa, dvv, red5 = tmix_mid_backward(
             k, v, vf2, ww, aa, vv, w0.reshape(C), a0.reshape(C), v0.reshape(C) if has_vres else None, k_k.reshape(C),

@@ -49,48 +49,79 @@ def _flags(bounded_decay, chunk_checkpoints, tf32=False):
                          (TF32 if (tf32 and bounded_decay) else 0))
 
 
-def forward_raw(w, q, k, v, a, b, bounded_decay: bool = False, chunk_checkpoints: bool = False, tf32: bool = False):
+def cache_bytes(B: int, T: int, H: int) -> int:
+    """Size of the chunk cache of forward_raw(..., chunk_cache=True): 64 KB per 64-step chunk of each (batch, head)."""
+    L = _lib.lib()
+    L.vrwkv_wkv7_cache_bytes.restype = ctypes.c_size_t
+    return int(L.vrwkv_wkv7_cache_bytes(B, T, H))
+
+
+def forward_raw(w, q, k, v, a, b, bounded_decay: bool = False, chunk_checkpoints: bool = False, tf32: bool = False,
+                chunk_cache: bool = False):
     """[B,T,H,64] bf16 x6 (kernel order) -> y, s, sa through the C ABI (vrwkv_wkv7_forward_ex).
 
     bounded_decay=True is the caller's promise that exp(w) <= 0.607 (RWKV-7's w = -softplus(.) - 0.5, model.py:176);
     it lets the library use the chunked tensor-core kernels.  chunk_checkpoints=True (needs bounded_decay, T % 64 == 0):
-    s is [B,H,T/64,64,64], one state per chunk — pass the same to backward_raw."""
+    s is [B,H,T/64,64,64], one state per chunk — pass the same to backward_raw.  chunk_cache=True (needs both, not
+    tf32): returns y, s, sa, cache, where cache (uint8, cache_bytes(B, T, H)) holds what the forward computed per
+    chunk and the backward would otherwise recompute — pass it to backward_raw(..., cache=cache)."""
     L = _lib.lib()
     B, T, H, C = w.shape
     assert C == 64 and T % CHUNK_LEN == 0
     assert all(i.dtype == torch.bfloat16 and i.is_contiguous() and i.is_cuda for i in [w, q, k, v, a, b])
     y = torch.empty_like(v)
     chunk_checkpoints = bool(chunk_checkpoints and bounded_decay and T % CHUNK == 0)
+    if chunk_cache and not (chunk_checkpoints and not tf32):
+        raise ValueError("chunk_cache needs bounded_decay, chunk_checkpoints, T % 64 == 0 and not tf32")
     s = torch.empty(B, H, T // (CHUNK if chunk_checkpoints else CHUNK_LEN), C, C, dtype=torch.float32, device=w.device)
     sa = torch.empty(B, T, H, C, dtype=torch.float32, device=w.device)
+    cache = torch.empty(cache_bytes(B, T, H), dtype=torch.uint8, device=w.device) if chunk_cache else None
 
     def run():
         with torch.cuda.device(w.device):
-            rc = L.vrwkv_wkv7_forward_ex(B, T, H, _lib.ptr(w), _lib.ptr(q), _lib.ptr(k), _lib.ptr(v), _lib.ptr(a),
-                                         _lib.ptr(b), _lib.ptr(y), _lib.ptr(s), _lib.ptr(sa), None, None,
-                                         _flags(bounded_decay, chunk_checkpoints, tf32), _lib.cur_stream())
-        _lib.check(rc, "vrwkv_wkv7_forward_ex")
+            if chunk_cache:
+                rc = L.vrwkv_wkv7_forward_cache(B, T, H, _lib.ptr(w), _lib.ptr(q), _lib.ptr(k), _lib.ptr(v), _lib.ptr(a),
+                                                _lib.ptr(b), _lib.ptr(y), _lib.ptr(s), _lib.ptr(sa), _lib.ptr(cache),
+                                                _flags(True, True), _lib.cur_stream())
+            else:
+                rc = L.vrwkv_wkv7_forward_ex(B, T, H, _lib.ptr(w), _lib.ptr(q), _lib.ptr(k), _lib.ptr(v), _lib.ptr(a),
+                                             _lib.ptr(b), _lib.ptr(y), _lib.ptr(s), _lib.ptr(sa), None, None,
+                                             _flags(bounded_decay, chunk_checkpoints, tf32), _lib.cur_stream())
+        _lib.check(rc, "vrwkv_wkv7_forward_cache" if chunk_cache else "vrwkv_wkv7_forward_ex")
 
     _timed("fwd", run)
-    return y, s, sa
+    return (y, s, sa, cache) if chunk_cache else (y, s, sa)
 
 
-def backward_raw(w, q, k, v, a, b, dy, s, sa, bounded_decay: bool = False, tf32: bool = False):
+def backward_raw(w, q, k, v, a, b, dy, s, sa, bounded_decay: bool = False, tf32: bool = False, cache=None):
     """Returns dw, dq, dk, dv, da, db (bf16 [B,T,H,64]) through vrwkv_wkv7_backward_ex (the checkpoint granularity is
-    read off the shape of s)."""
+    read off the shape of s), or through vrwkv_wkv7_backward_cache when given the cache of forward_raw(...,
+    chunk_cache=True)."""
     L = _lib.lib()
     B, T, H, C = w.shape
     chunk_checkpoints = s.shape[2] * CHUNK == T and s.shape[2] * CHUNK_LEN != T
     assert dy.dtype == torch.bfloat16 and dy.is_contiguous()
+    if cache is not None:
+        if not (bounded_decay and chunk_checkpoints and not tf32):
+            raise ValueError("cache needs bounded_decay, 64-step checkpoints and not tf32")
+        if (cache.dtype != torch.uint8 or cache.dim() != 1 or cache.numel() != cache_bytes(B, T, H)
+                or not cache.is_contiguous() or cache.device != w.device):
+            raise ValueError(f"cache must be a contiguous uint8 tensor of {cache_bytes(B, T, H)} bytes on {w.device}, "
+                             f"got {cache.dtype} {tuple(cache.shape)} on {cache.device}")
     outs = [torch.empty_like(w) for _ in range(6)]
 
     def run():
         with torch.cuda.device(w.device):
-            rc = L.vrwkv_wkv7_backward_ex(B, T, H, _lib.ptr(w), _lib.ptr(q), _lib.ptr(k), _lib.ptr(v), _lib.ptr(a),
-                                          _lib.ptr(b), _lib.ptr(dy), _lib.ptr(s), _lib.ptr(sa),
-                                          *[_lib.ptr(o) for o in outs],
-                                          _flags(bounded_decay, chunk_checkpoints, tf32), _lib.cur_stream())
-        _lib.check(rc, "vrwkv_wkv7_backward_ex")
+            if cache is not None:
+                rc = L.vrwkv_wkv7_backward_cache(B, T, H, _lib.ptr(w), _lib.ptr(q), _lib.ptr(k), _lib.ptr(v), _lib.ptr(a),
+                                                 _lib.ptr(b), _lib.ptr(dy), _lib.ptr(s), _lib.ptr(sa), _lib.ptr(cache),
+                                                 *[_lib.ptr(o) for o in outs], _flags(True, True), _lib.cur_stream())
+            else:
+                rc = L.vrwkv_wkv7_backward_ex(B, T, H, _lib.ptr(w), _lib.ptr(q), _lib.ptr(k), _lib.ptr(v), _lib.ptr(a),
+                                              _lib.ptr(b), _lib.ptr(dy), _lib.ptr(s), _lib.ptr(sa),
+                                              *[_lib.ptr(o) for o in outs],
+                                              _flags(bounded_decay, chunk_checkpoints, tf32), _lib.cur_stream())
+        _lib.check(rc, "vrwkv_wkv7_backward_cache" if cache is not None else "vrwkv_wkv7_backward_ex")
 
     _timed("bwd", run)
     return outs
